@@ -71,7 +71,29 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sort", action="store_true")
     ap.add_argument("--static-map", action="store_true", help="static balanced snapshot instead of the live ikd-Tree")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step to DIR/<name>.npy (float32/float64), "
+                         "so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path's outputs (--impl ours)")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """One .npy per output, float32 or float64; integer outputs go to float64 (exact for the values they hold)."""
+    conv = {k: (a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in conv.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(a))
 
 
 # ------------------------------------------------------------------ clocks sampler (recipe's nvidia-smi line)
@@ -188,8 +210,7 @@ def cpu_reference_run(case, tree, steps: int, warmup: int, threads: int):
         orc.set_knn_ref(tree)
         kind = "reference-knn+port"
     else:
-        from malio_b200 import plugin
-        snap = plugin.build_static_snapshot(case.map_xyz, case.map_normal_y)
+        snap = po.build_static_snapshot(case.map_xyz, case.map_normal_y)
         orc.set_map_snapshot(snap.nodes, snap.node_cov)
         kind = "port"
     times, passes = [], 0
@@ -328,7 +349,7 @@ def run_ours_c5(args, rank, world):
         sampler.start()
     for _ in range(max(args.warmup, 3)):
         m.Nearest_Search(q)
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     c0 = m.counters()
     dev_ms, e2e_ms = [], []
     tw0 = time.time()
@@ -343,6 +364,10 @@ def run_ours_c5(args, rank, world):
         e1.record(); torch.cuda.synchronize()
         dev_ms.append(ms); e2e_ms.append(e0.elapsed_time(e1))
     tw1 = time.time()
+    if args.dump_outputs and rank == 0:
+        # a fixed sample of rank 0's queries keeps the dump small (1M x 5 lists would be 60 MB)
+        pick = np.sort(np.random.default_rng(0).choice(idx.shape[0], min(idx.shape[0], 100_000), replace=False))
+        dump_outputs(args.dump_outputs, {"knn_query_index": pick + lo, "knn_idx": idx[pick], "knn_sqdist": d2[pick]})
     c1 = m.counters()
     clocks = sampler.stop(tw0, tw1) if rank == 0 else None
     t = torch.tensor([float(np.sum(dev_ms)), float(np.sum(e2e_ms))], device="cuda", dtype=torch.float64)
@@ -447,7 +472,7 @@ def run_ours(args, rank, world):
     def step_resident():
         model.rearm_scan()
         x, P = case.x_prop.copy(), case.P_prop.copy()
-        return model.update_iterated_dyn_share_modified(x, P, case.max_iter), x
+        return model.update_iterated_dyn_share_modified(x, P, case.max_iter), x, P
 
     # root box of the map = the ikd-Tree root's node_range_* (node 0's point + its two children's boxes)
     n0 = snap.nodes[0]
@@ -625,6 +650,17 @@ def run_ours(args, rank, world):
     model.set_timing(False)       # no per-pass event records inside the measured loops
     tot_ms, reps, c0, c1, out, (tw0, tw1) = timed(step_resident, args.steps, args.warmup)
     x_res = out[1]
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed step receives: the updated state and covariance, the report's deterministic fields and the
+        # per-point side outputs of the last pass (rank 0's block of the scan when sharded); written after all timing
+        rep_last, x_last, P_last = out
+        aux = model.aux()
+        dumped = {"state": synth.state_to_vec(x_last, case.n_lidar), "P": P_last, "dx_last": np.array(rep_last.dx_last[: case.n_dof]),
+                  "report": np.array([rep_last.passes, rep_last.searches, rep_last.converged_count, rep_last.last_status,
+                                      rep_last.n_eff_last], np.float64),
+                  "normal_y": aux["normal_y"], "nn_idx": aux["nn_idx"], "nn_sqdist": aux["nn_sqdist"], "selected": aux["selected"],
+                  "world": aux["world"]}
     passes = sum(r.passes for r in reps)
     searches = sum(r.searches for r in reps)
     launches = int(c1.kernel_launches - c0.kernel_launches)
@@ -797,6 +833,8 @@ def run_ours(args, rank, world):
             "what": "rank 0, %globaltimer inside pass_kernel: push of this GPU's keys / system to every peer + wait for all of theirs; the "
                     "MIN exchange is where a rank waits for the slowest rank to have launched its pass (host launch skew)"}
     print(json.dumps(line))
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     model.close()
     if tree is not None:
         with c_stdout_to_stderr():

@@ -761,6 +761,47 @@ void orc_knn_snapshot_batch(const malio_map_node* nodes, const float* cov, uint3
   if (visits_total) *visits_total = vt;
 }
 
+// Balanced snapshot over a static point set: median split on the longest extent (KD_TREE::BuildTree,
+// ikd_Tree.cpp:696-735), written straight in snapshot form.  The CPU arm of bench.py maps this instead of the
+// product's malio_build_static_snapshot when no live reference tree was built; same rule, same nth_element,
+// so the same snapshot (tests/test_oracle_cpu.py checks both byte for byte).
+static void static_build_rec(const float* xyz, uint32_t* order, int64_t l, int64_t r, uint32_t slot, uint32_t depth,
+                             malio_map_node* out, uint32_t* order_out, float box[6], uint32_t& max_depth) {
+  max_depth = std::max(max_depth, depth);
+  float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
+  for (int64_t i = l; i <= r; ++i) {
+    const float* p = xyz + 3 * (size_t)order[i];
+    for (int k = 0; k < 3; ++k) { mn[k] = std::min(mn[k], p[k]); mx[k] = std::max(mx[k], p[k]); }
+  }
+  int axis = 0;
+  for (int k = 1; k < 3; ++k) if (mx[k] - mn[k] > mx[axis] - mn[axis]) axis = k;
+  const int64_t mid = (l + r) >> 1;
+  std::nth_element(order + l, order + mid, order + r + 1,
+                   [&](uint32_t a, uint32_t b) { return xyz[3 * (size_t)a + axis] < xyz[3 * (size_t)b + axis]; });
+  malio_map_node& o = out[slot];
+  const float* p = xyz + 3 * (size_t)order[mid];
+  o.x = p[0]; o.y = p[1]; o.z = p[2];
+  order_out[slot] = order[mid];
+  const int64_t nl = mid - l, nr = r - mid;
+  o.link = (nl > 0 ? MALIO_LINK_HAS_LEFT : 0u) | (nr > 0 ? (MALIO_LINK_HAS_RIGHT | (uint32_t)(slot + 1 + nl)) : 0u);
+  for (int k = 0; k < 6; ++k) { o.lbox[k] = 0.f; o.rbox[k] = 0.f; }
+  for (int k = 0; k < 3; ++k) { box[2 * k] = mn[k]; box[2 * k + 1] = mx[k]; }
+  if (nl > 0) static_build_rec(xyz, order, l, mid - 1, slot + 1, depth + 1, out, order_out, o.lbox, max_depth);
+  if (nr > 0) static_build_rec(xyz, order, mid + 1, r, (uint32_t)(slot + 1 + nl), depth + 1, out, order_out, o.rbox, max_depth);
+}
+
+int orc_build_static_snapshot(const float* xyz, uint32_t n, malio_map_node* nodes_out, uint32_t* order_out, uint32_t* max_depth_out) {
+  uint32_t md = 0;
+  if (n > 0) {
+    std::vector<uint32_t> order(n);
+    for (uint32_t i = 0; i < n; ++i) order[i] = i;
+    float box[6];
+    static_build_rec(xyz, order.data(), 0, (int64_t)n - 1, 0, 1, nodes_out, order_out, box, md);
+  }
+  *max_depth_out = md;
+  return 0;
+}
+
 // per-point pieces exported for unit tests
 int orc_esti_plane(const float* near4, float threshold, double cov_threshold, float pabcd[4], double* plane_cov) {
   return esti_plane(pabcd, near4, threshold, *plane_cov, cov_threshold) ? 1 : 0;

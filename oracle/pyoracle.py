@@ -75,6 +75,7 @@ def oracle_lib() -> C.CDLL:
         L.orc_voxel_grid.restype = C.c_int64
         L.orc_voxel_grid.argtypes = [vp, C.c_int64, C.c_float, vp, C.c_int64, vp]
         L.orc_update_iterated.argtypes = [vp, C.POINTER(capi.State), vp, C.c_int, C.c_double, C.c_int, vp, vp, C.POINTER(capi.UpdateReport)]
+        L.orc_build_static_snapshot.argtypes = [vp, C.c_uint32, vp, vp, C.POINTER(C.c_uint32)]
         _orc = L
     return _orc
 
@@ -281,6 +282,22 @@ def knn_snapshot(nodes, cov, q, k=5, nthreads=1):
     L.orc_knn_snapshot_batch(ptr(nodes), ptr(cov), nodes.shape[0], ptr(q), n, k, ptr(ids), ptr(d2), ptr(found),
                              C.byref(visits), nthreads, None)
     return ids, d2, found, int(visits.value)
+
+
+def build_static_snapshot(xyz, normal_y=0.001):
+    """The static balanced snapshot of plugin.build_static_snapshot without mapping the product library."""
+    from malio_b200 import plugin
+    xyz = np.ascontiguousarray(xyz, np.float32)
+    n = xyz.shape[0]
+    nodes = np.zeros(n, dtype=capi.MAP_NODE)
+    order = np.zeros(n, dtype=np.uint32)
+    depth = C.c_uint32(0)
+    oracle_lib().orc_build_static_snapshot(ptr(xyz), n, ptr(nodes), ptr(order), C.byref(depth))
+    if np.isscalar(normal_y):
+        cov = np.full(n, normal_y, dtype=np.float32)
+    else:
+        cov = np.ascontiguousarray(np.asarray(normal_y, dtype=np.float32)[order])
+    return plugin.MapSnapshot(nodes, cov, order.astype(np.int64), int(depth.value))
 
 
 class Oracle:

@@ -9,12 +9,13 @@ Checked, every point:
   * world points bit-identical, selection flags identical, N_eff identical, min/max keys equal;
   * the reduced system <= 1e-9 relative;
   * the full iterated update: same number of passes and searches, same N_eff in the last pass, selection flags and neighbour
-    lists after the last pass identical, state <= 1e-4 (north_star; measured ~1e-10), covariance <= 1e-6 relative."""
+    lists after the last pass identical, state <= 1e-4 (north_star; measured ~1e-10), covariance <= 1e-6 relative.
+Where oracle/_ref is not built, the same checks run on the product's static snapshot of the map, without the comparison
+with the real Nearest_Search (tests/test_oracle_cpu.py makes that one on the churned tree stored in tests/golden/)."""
 import numpy as np
 import pytest
 
 import helpers as H
-import pyoracle as po
 from malio_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -25,11 +26,9 @@ P_TOL = 1e-6
 
 
 def _full_parity(case, threads=16):
-    if not po.ref_available():
-        pytest.skip("oracle/_ref (the real ikd_Tree.cpp) was not built")
     L = case.n_lidar
     snap, tree = H.snapshot_for(case, churn=True)
-    assert (snap.nodes["link"] & 0x20000000).any(), "the churned tree must carry deleted points"
+    assert tree is None or (snap.nodes["link"] & 0x20000000).any(), "the churned tree must carry deleted points"
     model = H.make_model(case, snap)
     orc = H.make_oracle(case, snap)
 
@@ -45,12 +44,12 @@ def _full_parity(case, threads=16):
     assert np.array_equal(gi, ao["nn_idx"].astype(np.int64)), "k-NN index lists must be bit-exact (restated Search)"
     found5 = ao["nn_cnt"] == 5
     assert np.array_equal(ag["nn_sqdist"][found5], ao["nn_sqdist"][found5])
-    # ... and against the real reference tree: ids through the snapshot's slot -> point id map
-    r_ids, r_d2, _, r_found = tree.knn(ag["world"], nthreads=threads)
-    mapped = np.where(gi >= 0, snap.node_ids[np.where(gi >= 0, gi, 0)], -1)
-    assert np.array_equal((gi >= 0).sum(1), r_found)
-    assert np.array_equal(mapped, r_ids.astype(np.int64)), "k-NN index lists must be bit-exact (real Nearest_Search)"
-    assert np.array_equal(ag["nn_sqdist"][found5], r_d2[found5])
+    if tree is not None:   # ... and against the real reference tree: ids through the snapshot's slot -> point id map
+        r_ids, r_d2, _, r_found = tree.knn(ag["world"], nthreads=threads)
+        mapped = np.where(gi >= 0, snap.node_ids[np.where(gi >= 0, gi, 0)], -1)
+        assert np.array_equal((gi >= 0).sum(1), r_found)
+        assert np.array_equal(mapped, r_ids.astype(np.int64)), "k-NN index lists must be bit-exact (real Nearest_Search)"
+        assert np.array_equal(ag["nn_sqdist"][found5], r_d2[found5])
     assert np.array_equal(ag["selected"], ao["selected"])
     assert st.n_eff == so.n_eff and st.n_eff > 0.5 * case.pts.shape[0]
     for a, b in ((st.u_min, so.u_min), (st.u_max, so.u_max), (st.tau_min, so.tau_min), (st.tau_max, so.tau_max)):
@@ -78,7 +77,9 @@ def _full_parity(case, threads=16):
     gi = ag["nn_idx"].astype(np.int64)
     gi[gi == 0xFFFFFFFF] = -1
     assert np.array_equal(gi, ao["nn_idx"].astype(np.int64)), "Nearest_Points after the last search"
-    model.close(); orc.close(); tree.close()
+    model.close(); orc.close()
+    if tree is not None:
+        tree.close()
     return d_state
 
 

@@ -5,21 +5,26 @@ include/malio_mapsync.hpp).  Checked: after every scan the device's live set is 
 10 scans the k-NN lists of 20k queries equal those of a FULL re-upload of the tree's snapshot (exact tree mode) — float
 distances bit-identical everywhere, index lists identical except where two neighbours are at exactly tied distances (the
 reference breaks those by traversal order; counted, SURVEY.md §7); a whole measurement pass agrees; H2D stays
-proportional to the changed points."""
+proportional to the changed points.
+Where oracle/_ref is not built, the device replays the tree's recorded answers to the stream of tests/test_mapops_cpu.py
+(tests/golden/), and the full re-uploads are static snapshots of the same live points."""
 import numpy as np
 import pytest
 
 import helpers as H
 import pyoracle as po
 from malio_b200 import capi, plugin, synth
-from test_mapops_cpu import scripted_stream, same_set
+from test_mapops_cpu import live_set_digest, recorded_stream, same_set, scripted_stream
 
 pytestmark = pytest.mark.gpu
 
 
-def _check_knn(dev, tree, rng, n_q=20000):
-    nodes, cov, ids, depth, live = tree.snapshot()
-    snap = plugin.MapSnapshot(nodes, cov, ids, depth)
+def static_snapshot_of(xyz, ny, ids):
+    s = plugin.build_static_snapshot(xyz, ny)
+    return plugin.MapSnapshot(s.nodes, s.node_cov, np.asarray(ids)[s.node_ids], s.max_depth)
+
+
+def _check_knn(dev, snap, rng, n_q=20000):
     full = plugin.MeasurementModel(1)
     full.upload_map(snap)
     m = dev.map_download()
@@ -44,8 +49,39 @@ def _check_knn(dev, tree, rng, n_q=20000):
     return len(bad)
 
 
-@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref (the real ikd_Tree.cpp) was not built")
+def _replay_recorded_stream_on_the_device():
+    rng = np.random.default_rng(17)
+    dev = plugin.MeasurementModel(1)
+    ev0 = next(scripted_stream())
+    dev.map_build(ev0[1], ev0[2], ev0[3])
+    h2d0 = dev.counters().h2d_bytes
+    scans = 0
+    for ev, ndel, cnt, sync, valid, digest in recorded_stream():
+        _, a, ny, ids, b, ny2, ids2, boxes = ev
+        if boxes is not None:
+            assert ndel == dev.map_delete_boxes(boxes)
+        dev.map_sync_voxels(sync, want_count=(scans % 2 == 0))
+        if scans % 2:
+            for k in ("boxes", "xyz", "normal_y", "ids"):
+                sync[k][...] = 0
+        dev.map_add_points(b, ny2, ids2)
+        b[...] = 0
+        m = dev.map_download()
+        assert live_set_digest(m["xyz"], m["normal_y"], m["ids"]) == digest, scans
+        live, slots = dev.map_info()
+        assert live == valid
+        scans += 1
+        if scans % 10 == 0:
+            _check_knn(dev, static_snapshot_of(m["xyz"], m["normal_y"], m["ids"]), rng)
+    per_scan = (dev.counters().h2d_bytes - h2d0) / 50.0
+    assert per_scan < 5 * 20000 * 12 / 50.0 + 40000, per_scan
+    dev.close()
+
+
 def test_fifty_scan_delta_stream_tracks_the_real_tree():
+    if not po.ref_available():
+        _replay_recorded_stream_on_the_device()
+        return
     rng = np.random.default_rng(17)
     tree = po.RefTree(box_length=0.5)
     dev = plugin.MeasurementModel(1)
@@ -75,18 +111,22 @@ def test_fifty_scan_delta_stream_tracks_the_real_tree():
         assert live == tree.validnum()
         scans += 1
         if scans % 10 == 0:
-            _check_knn(dev, tree, rng)
+            nodes, cov, ids, depth, _ = tree.snapshot()
+            _check_knn(dev, plugin.MapSnapshot(nodes, cov, ids, depth), rng)
     per_scan = (dev.counters().h2d_bytes - h2d0) / 50.0
     # k-NN test queries are uploads too (5 x 20k x 12 B); what remains is the deltas: ~500 points + boxes per scan
     assert per_scan < 5 * 20000 * 12 / 50.0 + 40000, per_scan
     dev.close(); tree.close()
 
 
-@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref (the real ikd_Tree.cpp) was not built")
 def test_measurement_pass_on_the_device_resident_map_equals_snapshot_mode_and_compaction_keeps_it():
+    """Snapshot mode on the churned reference tree where oracle/_ref is built, else on the static snapshot of the map."""
     case = synth.make_case("mapmode", 20000, 200000, 3, 3)
     snap, tree = H.snapshot_for(case, churn=True)
-    fx, fny, fid = tree.flatten_points()
+    if tree is not None:
+        fx, fny, fid = tree.flatten_points()
+    else:
+        fx, fny, fid = case.map_xyz, case.map_normal_y, np.arange(case.map_xyz.shape[0], dtype=np.int32)
     ref = H.make_model(case, snap)                       # snapshot (tree) mode
     dev = plugin.MeasurementModel(3, params=case.params)  # device-resident map built from the same live points
     dev.map_build(fx, fny, fid)
@@ -114,11 +154,21 @@ def test_measurement_pass_on_the_device_resident_map_equals_snapshot_mode_and_co
     lo = fx.min(0); hi = fx.max(0)
     cut = lo[0] + 0.6 * (hi[0] - lo[0])
     box = np.array([[lo[0] - 1, lo[1] - 1, lo[2] - 1, cut, hi[1] + 1, hi[2] + 1]], np.float32)
-    assert tree.delete_boxes(box) == dev.map_delete_boxes(box)
-    tree.wait_rebuild()
+    if tree is not None:
+        assert tree.delete_boxes(box) == dev.map_delete_boxes(box)
+        tree.wait_rebuild()
+        n_live = tree.validnum()
+        nodes, cov, ids, depth, _ = tree.snapshot()
+        survivors = plugin.MapSnapshot(nodes, cov, ids, depth)
+    else:
+        keep = ~np.all((box[0, :3] <= fx) & (box[0, 3:] > fx), axis=1)    # half-open boxes, as Delete_Point_Boxes
+        assert int((~keep).sum()) == dev.map_delete_boxes(box)
+        n_live = int(keep.sum())
+        survivors = static_snapshot_of(fx[keep], fny[keep], fid[keep])
     live, slots = dev.map_info()
-    assert live == slots == tree.validnum() and dev.counters().map_compactions == 1
-    nodes, cov, ids, depth, _ = tree.snapshot()
-    ref.upload_map(plugin.MapSnapshot(nodes, cov, ids, depth))
+    assert live == slots == n_live and dev.counters().map_compactions == 1
+    ref.upload_map(survivors)
     compare()
-    ref.close(); dev.close(); tree.close()
+    ref.close(); dev.close()
+    if tree is not None:
+        tree.close()

@@ -2,12 +2,19 @@
 The real reference ikd-Tree (oracle/_ref) and a flat numpy mirror receive the same 50-scan scripted stream of
 Add_Points (with and without down-sampling) / Delete_Point_Boxes; the mirror only ever sees what the device would see
 (appends, boxes, per-voxel re-synchronisation records collected through KD_TREE::Box_Search).  After every scan the
-mirror's live set must equal KD_TREE::flatten() point for point — whatever the tree's topology and re-build timing."""
+mirror's live set must equal KD_TREE::flatten() point for point — whatever the tree's topology and re-build timing.
+Where oracle/_ref is not built, the mirror replays the tree's answers to the same stream (tests/golden/make_ref_golden.py)."""
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
 import pyoracle as po
 import np_mapops as nm
+
+VOXEL = 0.5
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ikd_ref_golden.npz")
 
 
 def scripted_stream(seed=1, M=20000, scans=50):
@@ -32,6 +39,39 @@ def scripted_stream(seed=1, M=20000, scans=50):
         yield ("scan", a, ny, ids, b, np.full(60, 0.002, np.float32), ids2, boxes)
 
 
+def live_set_digest(xyz, ny, ids) -> bytes:
+    """SHA-256 of a live point set ordered by id: equal digests <=> equal sets, point for point."""
+    o = np.argsort(ids, kind="stable")
+    h = hashlib.sha256(np.asarray(ids, np.int64)[o].tobytes())
+    h.update(np.ascontiguousarray(xyz, np.float32)[o].tobytes())
+    h.update(np.ascontiguousarray(ny, np.float32)[o].tobytes())
+    return h.digest()
+
+
+def recorded_stream():
+    """The reference tree's answers to scripted_stream() (defaults), from the golden file: yields per scan
+    (event, Delete_Point_Boxes count, Add_Points count, sync record as add_points_synced returns it, validnum, live-set digest)."""
+    g = np.load(GOLD)
+    events = list(scripted_stream())
+    by_id = {}
+    for ev in events:
+        pairs = [(ev[1], ev[2], ev[3])] if ev[0] == "build" else [(ev[1], ev[2], ev[3]), (ev[4], ev[5], ev[6])]
+        for xyz, ny, ids in pairs:
+            by_id.update(zip(ids.tolist(), zip(xyz.copy(), ny.copy())))   # copies: callers may overwrite the event's arrays
+    ob = om = 0
+    for s, ev in enumerate(events[1:]):
+        nb = int(g["stream_nb"][s])
+        counts = g["stream_counts"][ob:ob + nb].astype(np.uint32)
+        m = int(counts.sum())
+        lo = g["stream_vox"][ob:ob + nb].astype(np.float32) * np.float32(VOXEL)
+        ids = g["stream_ids"][om:om + m]
+        sync = dict(boxes=np.concatenate([lo, lo + np.float32(VOXEL)], 1), counts=counts,
+                    xyz=np.array([by_id[i][0] for i in ids.tolist()], np.float32).reshape(-1, 3),
+                    normal_y=np.array([by_id[i][1] for i in ids.tolist()], np.float32), ids=ids.copy(), outside_own_box=0)
+        ob += nb; om += m
+        yield ev, int(g["stream_ndel"][s]), int(g["stream_added"][s]), sync, int(g["stream_valid"][s]), g["stream_digest"][s].tobytes()
+
+
 def same_set(tree, mirror):
     fx, fny, fid = tree.flatten_points()
     lx, lny, lid = mirror
@@ -41,9 +81,32 @@ def same_set(tree, mirror):
     return np.array_equal(fid[a], np.asarray(lid)[b]) and np.array_equal(fx[a], lx[b]) and np.array_equal(fny[a], lny[b])
 
 
-@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref (the real ikd_Tree.cpp) was not built")
+def _replay_recorded_stream():
+    mir = nm.MirrorMap()
+    ev0 = next(scripted_stream())
+    mir.build(ev0[1], ev0[2], ev0[3])
+    synced_pts = 0
+    for ev, ndel, cnt, sync, valid, digest in recorded_stream():
+        _, a, ny, ids, b, ny2, ids2, boxes = ev
+        if boxes is not None:
+            assert ndel == mir.delete_boxes(boxes)
+        assert cnt > 0
+        assert len(np.unique(sync["boxes"], axis=0)) == len(sync["boxes"])
+        mir.sync_voxels(sync)
+        synced_pts += len(sync["ids"])
+        mir.add_points(b, ny2, ids2)
+        live = mir.live_points()
+        assert len(live[2]) == valid and live_set_digest(*live) == digest
+    assert synced_pts < 50 * 400 * 3
+
+
 @pytest.mark.parametrize("threads", [1, 8])
 def test_delta_protocol_keeps_a_flat_mirror_equal_to_the_real_tree(threads):
+    """With oracle/_ref: the live tree, read back with `threads` threads.  Without: the recorded answers of that tree (collected
+    with 1 and with 8 threads, identical)."""
+    if not po.ref_available():
+        _replay_recorded_stream()
+        return
     tree = po.RefTree(box_length=0.5)
     mir = nm.MirrorMap()
     synced_pts = 0
